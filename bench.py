@@ -37,6 +37,7 @@ os.environ.setdefault("NCCL_DEBUG_FILE", "/dev/stderr")  # keep stdout to the on
 
 METRIC = "atoms/sec (energy+forces) CHGNet a-Si r_cut=5A"
 SURVEY_BYTES_PER_EDGE = 314.0  # SURVEY.md 8(d), rbf-recompute variant, D=64 fp32
+DUMP_BYTES = 60_000_000  # array bytes --dump-outputs writes at most: under 64 MB with the .npy headers
 
 
 def load_peaks():
@@ -220,6 +221,23 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(d, arrays):
+    """Write each array as d/<name>.npy, float32 kept, anything else as float64.  When the arrays come to more than
+    DUMP_BYTES, the largest (the forces) keeps a seeded, sorted sample of its rows: the same rows for the same
+    arguments, so that the dumps of two builds compare row for row."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in arrays.items()}
+    big = max(arrays, key=lambda k: arrays[k].nbytes)
+    rest = sum(v.nbytes for k, v in arrays.items() if k != big)
+    a = arrays[big]
+    if rest + a.nbytes > DUMP_BYTES:
+        keep = (DUMP_BYTES - rest) // (a.nbytes // len(a))
+        arrays[big] = a[np.sort(np.random.default_rng(0).choice(len(a), size=keep, replace=False))]
+    os.makedirs(d, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(d, f"{k}.npy"), v)
+
+
 def parity_block(atoms, out, pot_factory, rank, world, local, release=None):
     """Correctness evidence computed in the run (outside the timed region).  Always: net force, virial symmetry,
     energy per atom, checksum of the forces of 4096 seeded atoms.  At N > 1 rank 0 also evaluates the same cell on a
@@ -324,7 +342,7 @@ def run_ours(args):
     t0 = time.perf_counter()
     dev_ms, gather_ms, launches = 0.0, [], 0
     for _ in range(args.steps):
-        _e, ms = eng.compute_resident(1)
+        e_resident, ms = eng.compute_resident(1)
         dev_ms += ms
         gather_ms.append(eng.timings()["edge_gather_ms"])
         launches += eng.counts()["launches"]
@@ -355,6 +373,11 @@ def run_ours(args):
         dist.all_reduce(t2, op=dist.ReduceOp.MAX)
     e2e_ms = t2.item()
     e2e_val = natoms / (e2e_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # the last timed step of each loop: the energy compute_resident returns (forces and stress stay on the
+        # device there), and what Potential_Dist returns
+        dump_outputs(args.dump_outputs, {"resident_energy": np.float64(e_resident), "energy": out[0],
+                                         "forces": out[1], "stress": out[2]})
     c_final, tm = eng.counts(), eng.timings()
     parity = parity_block(atoms, out, single_partition_potential, rank, world, local, release=eng.release_workspace)
     barrier()
@@ -440,7 +463,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--model", default="chgnet", choices=["chgnet", "tensornet"],
                     help="tensornet: the SURVEY 8(f).2 path (reduced JSON line; the metric and the default are CHGNet)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy "
+                         "(resident_energy, energy, forces, stress; at most 64 MB, forces then a seeded sample of rows)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,11 +1,12 @@
-"""Generates tests/golden/graph_golden.json from the reference's own C graph builder (oracle/_ref,
-compiled from /root/reference by oracle/Makefile).  Run in the build container:
+"""Generates tests/golden/graph_golden.json and tests/golden/ref_edges_si_6x6x7_P2.npz from the reference's own
+C graph builder (oracle/_ref, compiled by oracle/Makefile from a DistMLIP checkout).  With that checkout at hand:
 
-    make -C oracle && python tests/golden/make_golden.py
+    make -C oracle REF=<DistMLIP checkout> && python tests/golden/make_golden.py
 
-Each case stores order-independent integer digests of what get_subgraphs_fast returned
-(subgraph_creation_fast.c:403-422), so the numpy restatement (oracle/graph_ref.py) and the CUDA graph
-builder can be checked without the reference being present (it does not exist on the GPU box).
+Each case of graph_golden.json stores order-independent integer digests of what get_subgraphs_fast returned
+(subgraph_creation_fast.c:403-422); the .npz stores one cell's edge set in full (see reference_edges).  With
+them the numpy restatement (oracle/graph_ref.py) and the CUDA graph builder are checked against the reference
+wherever the tests run, with or without a DistMLIP checkout.
 """
 import json
 import os
@@ -85,8 +86,44 @@ def describe(atoms, P):
     return d
 
 
+REF_EDGES = "ref_edges_si_6x6x7_P2.npz"
+
+
+def reference_edges(n_dist=4096):
+    """What tests/test_oracle.py::test_graph_oracle_matches_live_reference compares with, for
+    si_diamond(6, nz=7, seed=11) on 2 slabs: the whole edge set in canonical (i1, i2, off) order, the partition
+    that owns each edge, the halo lists, the number of angles of each partition, and the distances of a fixed
+    seeded sample of n_dist edges (all 56k of them would make the file five times larger)."""
+    atoms = si_diamond(6, nz=7, seed=11)
+    cart, lat, pbc = atoms.get_positions(), atoms.get_cell(), atoms.get_pbc().astype(np.int64)
+    t = G.ref_get_subgraphs(cart, atoms.get_scaled_positions(wrap=True), lat, pbc, 2, 5.0, 3.0, True)
+    c = G.canon_from_ref_tuple(t, 2)
+    order = np.lexsort((c["off"][:, 2], c["off"][:, 1], c["off"][:, 0], c["i2"], c["i1"]))
+    owner = np.full(len(order), -1, dtype=np.int8)
+    for p in range(2):
+        owner[t[16][p]] = p  # local -> global edge map of partition p
+    assert (owner >= 0).all()
+    i1, i2, off, owner = c["i1"][order], c["i2"][order], c["off"][order], owner[order]
+    dist_idx = np.sort(np.random.default_rng(0).choice(len(order), size=n_dist, replace=False))
+    out = {"i1": i1.astype(np.int32), "i2": i2.astype(np.int32), "off": off.astype(np.int8), "owner": owner,
+           "dist_idx": dist_idx.astype(np.int32), "dist": c["dist"][order][dist_idx],
+           "n_angles": np.array([len(c["parts"][p]["line_src"]) for p in range(2)], dtype=np.int64)}
+    for p in range(2):
+        for q in range(2):
+            out[f"to_{p}_{q}"] = np.asarray(c["parts"][p]["to"][q], dtype=np.int32)
+            out[f"from_{p}_{q}"] = np.asarray(c["parts"][p]["from"][q], dtype=np.int32)
+        # the owner mask restates the partition's canonically sorted edge list exactly
+        m = owner == p
+        po = np.lexsort((off[m, 2], off[m, 1], off[m, 0], i1[m], i2[m]))
+        s, d, _o = c["parts"][p]["edges"]
+        assert np.array_equal(i1[m][po], s) and np.array_equal(i2[m][po], d)
+    return out
+
+
 if __name__ == "__main__":
+    here = os.path.dirname(os.path.abspath(__file__))
     res = {k: describe(a, P) for k, (a, P) in cases().items()}
-    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "graph_golden.json"), "w") as f:
+    with open(os.path.join(here, "graph_golden.json"), "w") as f:
         json.dump(res, f, indent=1)
     print({k: (v["natoms"], v["edges"][0]) for k, v in res.items()})
+    np.savez_compressed(os.path.join(here, REF_EDGES), **reference_edges())

@@ -1,5 +1,5 @@
-import sys, time, numpy as np
-sys.path.insert(0, "/root/repo")
+import os, sys, time, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from distmlip_b200.structures import si_diamond
 from tests._util import make_model, engine_from_model
 m = make_model(); eng = engine_from_model(m)

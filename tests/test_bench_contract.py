@@ -43,6 +43,30 @@ def test_reference_arm_other_ranks_do_no_work():
     assert time.time() - t0 < 120
 
 
+def test_dump_outputs_keeps_a_fixed_sample_under_the_cap(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+
+    sys.path.insert(0, ROOT)
+    import importlib
+
+    bench = importlib.import_module("bench")
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 16)
+    f = np.arange(3 * 10000, dtype=np.float32).reshape(-1, 3)  # 120 kB of forces, row k = (3k, 3k+1, 3k+2)
+    arrays = {"resident_energy": np.float64(-1.5), "energy": torch.tensor(-1.5, dtype=torch.float64),
+              "forces": torch.from_numpy(f), "stress": torch.zeros(3, 3), "n": np.arange(4)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    got = {k: np.load(tmp_path / "a" / f"{k}.npy") for k in arrays}
+    assert all(v.dtype in (np.float32, np.float64) for v in got.values())
+    assert sum(v.nbytes for v in got.values()) <= 1 << 16
+    rows = got["forces"]
+    assert rows.dtype == np.float32 and 0 < len(rows) < len(f)
+    assert np.array_equal(rows, f[(rows[:, 0] / 3).astype(np.int64)]) and np.all(np.diff(rows[:, 0]) > 0)
+    assert np.array_equal(rows, np.load(tmp_path / "b" / "forces.npy"))
+    assert float(got["energy"]) == -1.5 and got["stress"].shape == (3, 3) and np.array_equal(got["n"], np.arange(4))
+
+
 def test_clock_sampler_windows(tmp_path, monkeypatch):
     fake = tmp_path / "nvidia-smi"
     fake.write_text("#!/bin/bash\nsleep 0.2\nwhile true; do echo '0, 1965, 1965, 500.1, 0x0, Not Active, Not Active, "
