@@ -18,6 +18,7 @@ SYMBOLS = [
     "b2m_finalize_weights", "b2m_set_scaling", "b2m_comm_unique_id", "b2m_comm_init", "b2m_set_partition", "b2m_set_structure", "b2m_compute",
     "b2m_compute_resident", "b2m_get_sitewise", "b2m_get_counts", "b2m_get_partition_info",
     "b2m_debug_tensor", "b2m_last_timings", "b2m_release_workspace", "b2m_set_view", "b2m_create_tensornet",
+    "b2m_compute_peratom",
 ]
 
 
@@ -73,6 +74,7 @@ def load_library():
     lib.b2m_set_partition.argtypes = [vp, i32, i32]
     lib.b2m_set_structure.argtypes = [vp, i64, P(dbl), P(dbl), P(C.c_int32), P(C.c_int), dbl]
     lib.b2m_compute.argtypes = [vp, i32, i32, P(dbl), P(C.c_float), P(C.c_float)]
+    lib.b2m_compute_peratom.argtypes = [vp, i32, P(dbl), P(C.c_float), P(C.c_float), P(dbl), P(C.c_float)]
     lib.b2m_compute_resident.argtypes = [vp, i32, i32, i32, P(dbl), P(C.c_float)]
     lib.b2m_get_sitewise.argtypes = [vp, P(C.c_float)]
     lib.b2m_get_counts.argtypes = [vp, P(i64), i32]
@@ -196,6 +198,21 @@ class Engine:
         sp = s.ctypes.data_as(C.POINTER(C.c_float)) if s is not None else None
         self._ck(self.lib.b2m_compute(self.h, int(bool(forces)), int(bool(stress)), C.byref(e), fp, sp))
         return e.value, f, (s.reshape(3, 3) if s is not None else None)
+
+    def compute_peratom(self, forces=True):
+        """compute() plus per-atom output of the same evaluation: (E, F or None, stress [3,3] GPa, atom_e [N] eV,
+        atom_W [N,3,3] eV).  sum(atom_e) == E and atom_W.sum(0) * 160.21766208 / V == stress (include/b200mlip.h)."""
+        e = C.c_double()
+        f = np.empty((self.natoms, 3), dtype=np.float32) if forces else None
+        s = np.empty(9, dtype=np.float32)
+        ae = np.empty(self.natoms, dtype=np.float64)
+        aw = np.empty((self.natoms, 9), dtype=np.float32)
+        fp = f.ctypes.data_as(C.POINTER(C.c_float)) if f is not None else None
+        self._ck(self.lib.b2m_compute_peratom(self.h, int(bool(forces)), C.byref(e), fp,
+                                              s.ctypes.data_as(C.POINTER(C.c_float)),
+                                              ae.ctypes.data_as(C.POINTER(C.c_double)),
+                                              aw.ctypes.data_as(C.POINTER(C.c_float))))
+        return e.value, f, s.reshape(3, 3), ae, aw.reshape(-1, 3, 3)
 
     def compute_resident(self, reps=1, forces=True, stress=True):
         e = C.c_double()

@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libb200mlip.so")
 SOURCES = ["graph.cu", "kernels.cu", "kernels_tc.cu", "kernels_ac3.cu", "kernels_tn.cu", "engine.cu"]
-HEADERS = ["common.cuh", "graph.cuh", "kernels.cuh", "tc_common.cuh", "tn_state.cuh", "engine_tn.inl", os.path.join("..", "..", "include", "b200mlip.h")]
+HEADERS = ["common.cuh", "graph.cuh", "kernels.cuh", "tc_common.cuh", "tn_state.cuh", "peratom.cuh", "engine_tn.inl", os.path.join("..", "..", "include", "b200mlip.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "--extended-lambda",
     "-Xcompiler", "-fPIC", "-Wno-deprecated-declarations",

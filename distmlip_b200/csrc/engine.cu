@@ -165,6 +165,11 @@ struct b2m_engine {
   std::vector<DBuf<float>> x, h, ang, upd, uv, uvB, dsB, uvA;
   DBuf<float> be_e, dbe_e;  // [E,12] radial basis and derivative, once per step
   bool want_grads = true;
+  // per-atom output (b2m_compute_peratom): W_i rows [N][kAtomVirW] f32 and e_i [N] f64 in global order, allocated on the
+  // first per-atom evaluation only; reduced over the partitions like `forces`
+  bool want_peratom = false;
+  DBuf<float> atom_vir, avtmp;  // avtmp / aetmp: leader's staging of a peer partition's arrays
+  DBuf<double> atom_e, aetmp;
   // first-layer projections of every atom-conv layer (A = x W1s^T, C = x W1t^T + b1, Q = h W1e^T), one buffer per
   // layer: the backward gathers the rows the forward wrote instead of re-running three GEMMs per layer
   // (about 1.1 GB per 100k atoms for the four layers)
@@ -922,13 +927,15 @@ static void backward(b2m_engine* e) {
   // geometry: h0 = W_be be(d_b), theta/Fourier, then edges -> forces and virial
   launch_h0_bwd(e->st, g.B_loc, g.b_vec.p, e->rp2, e->d_Wbe, e->gh.p, e->gdb.p);
   launch_angle_init_bwd(e->st, g.A, g.a_in.p, g.a_out.p, g.b_vec.p, e->d_fa, e->d_Wae, e->gang.p, e->gbvec.p, e->use_tc);
+  float* atom_vir = e->want_peratom ? e->atom_vir.p : nullptr;
   launch_edge_final(e->st, g.E, g.e_src.p, g.e_dst.p, g.e_bond.p, g.e_vec.p, g.gid.p, e->gd.p, e->gdb.p, e->gbvec.p,
-                    e->forces.p, e->scal.p + 1);
+                    e->forces.p, e->scal.p + 1, atom_vir);
   launch_halo_bond_final(e->st, g.B_own, g.B_loc, g.b_src_gid.p, g.b_dst.p, g.b_vec.p, g.gid.p, e->gdb.p, e->gbvec.p,
-                         e->forces.p, e->scal.p + 1);
+                         e->forces.p, e->scal.p + 1, atom_vir);
 }
 
-static void run(b2m_engine* e, bool grads) {
+// peratom (needs grads): also the per-atom energies and virials of this partition's owned rows and edges
+static void run(b2m_engine* e, bool grads, bool peratom = false) {
   B2M_REQUIRE(e->finalized, B2M_ERR_STATE, "weights not finalized");
   B2M_REQUIRE(e->have_graph, B2M_ERR_STATE, "b2m_set_structure has not been called");
   B2M_REQUIRE(e->world == 1 || e->comm != nullptr || e->leader != nullptr || e->debug_no_halo, B2M_ERR_STATE,
@@ -942,15 +949,29 @@ static void run(b2m_engine* e, bool grads) {
   const long long l0 = g_launch_count;
   B2M_CK(cudaEventRecord(e->ev[0], e->st));
   e->want_grads = grads;
+  e->want_peratom = peratom;
+  const size_t N = (size_t)e->g.N;
+  if (peratom) {
+    B2M_REQUIRE(grads, B2M_ERR_INVALID, "per-atom virials need the backward pass");
+    e->atom_vir.ensure(N * kAtomVirW), e->atom_e.ensure(N);
+    e->atom_vir.zero(N * kAtomVirW, e->st), e->atom_e.zero(N, e->st);
+  }
   if (e->kind == 1) tn_forward(e); else forward(e);
   B2M_CK(cudaEventRecord(e->ev[1], e->st));
   if (grads) {
     if (e->kind == 1) tn_backward(e); else backward(e);
   }
+  if (peratom)
+    launch_atom_energy(e->st, e->g.n_own, e->kind == 1 ? e->tn->e_atom.p : e->e_atom.p, e->g.gid.p, e->g.type.p,
+                       e->d_eref, (float)e->desc.data_std, e->desc.data_mean / (double)N, e->atom_e.p);
   if (e->world > 1 && e->leader == nullptr && !e->debug_no_halo) {
     NCCL_CK(g_nccl.AllReduce(e->scal.p, e->scal.p, 10, ncclFloat64, ncclSum, e->comm, e->st));
     if (grads)
       NCCL_CK(g_nccl.AllReduce(e->forces.p, e->forces.p, (size_t)e->g.N * 3, ncclFloat32, ncclSum, e->comm, e->st));
+    if (peratom) {
+      NCCL_CK(g_nccl.AllReduce(e->atom_vir.p, e->atom_vir.p, N * kAtomVirW, ncclFloat32, ncclSum, e->comm, e->st));
+      NCCL_CK(g_nccl.AllReduce(e->atom_e.p, e->atom_e.p, N, ncclFloat64, ncclSum, e->comm, e->st));
+    }
   }
   B2M_CK(cudaEventRecord(e->ev[2], e->st));
   B2M_CK(cudaStreamSynchronize(e->st));
@@ -995,7 +1016,8 @@ static void ensure_pinned(void*& p, size_t& cap, size_t bytes) {
   cap = bytes + bytes / 8;
 }
 
-__global__ void k_add_inplace(int64_t n, const float* __restrict__ src, float* __restrict__ dst) {
+template <class T>
+__global__ void k_add_inplace(int64_t n, const T* __restrict__ src, T* __restrict__ dst) {
   const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (i < n) dst[i] += src[i];
 }
@@ -1031,12 +1053,12 @@ static void for_each_part(b2m_engine* L, F fn) {
     if (codes[p] != 0) throw Error(codes[p], errs[p]);
 }
 
-static void run_any(b2m_engine* e, bool grads) {
+static void run_any(b2m_engine* e, bool grads, bool peratom = false) {
   if (e->parts.empty()) {
-    run(e, grads);
+    run(e, grads, peratom);
     return;
   }
-  for_each_part(e, [&](b2m_engine* pe) { run(pe, grads); });
+  for_each_part(e, [&](b2m_engine* pe) { run(pe, grads, peratom); });
   // slowest partition = the group's device time; launches summed
   long long launches = 0;
   for (auto* pe : e->parts) {
@@ -1078,6 +1100,28 @@ static void fetch(b2m_engine* e, double* energy, float* forces, float* stress9) 
   if (energy) *energy = e->last_energy;
   if (stress9)
     for (int k = 0; k < 9; k++) stress9[k] = (float)(hs[1 + k] / e->g.volume * 160.21766208);  // pes.py:140-145
+}
+
+// after fetch of a per-atom run: e_i [N] (eV) and W_i [N][9] (eV), global order
+static void fetch_peratom(b2m_engine* e, double* atom_energy, float* atom_virial9) {
+  const size_t n = (size_t)e->g.N, nw = n * kAtomVirW;
+  for (size_t p = 1; p < e->parts.size(); p++) {  // group: sum the partitions' arrays on the leader's device, as fetch
+    b2m_engine* pe = e->parts[p];                  // does the forces
+    e->avtmp.ensure(nw), e->aetmp.ensure(n);
+    B2M_CK(cudaMemcpyAsync(e->avtmp.p, pe->atom_vir.p, nw * sizeof(float), cudaMemcpyDefault, e->st));
+    k_add_inplace<<<cdiv((int64_t)nw, 256), 256, 0, e->st>>>((int64_t)nw, e->avtmp.p, e->atom_vir.p);
+    B2M_CK(cudaGetLastError());
+    B2M_CK(cudaMemcpyAsync(e->aetmp.p, pe->atom_e.p, n * sizeof(double), cudaMemcpyDefault, e->st));
+    k_add_inplace<<<cdiv((int64_t)n, 256), 256, 0, e->st>>>((int64_t)n, e->aetmp.p, e->atom_e.p);
+    B2M_CK(cudaGetLastError());
+  }
+  std::vector<float> rows(atom_virial9 ? nw : 0);
+  if (atom_energy) B2M_CK(cudaMemcpyAsync(atom_energy, e->atom_e.p, n * sizeof(double), cudaMemcpyDeviceToHost, e->st));
+  if (atom_virial9)
+    B2M_CK(cudaMemcpyAsync(rows.data(), e->atom_vir.p, nw * sizeof(float), cudaMemcpyDeviceToHost, e->st));
+  B2M_CK(cudaStreamSynchronize(e->st));
+  if (atom_virial9)
+    for (size_t i = 0; i < n; i++) memcpy(atom_virial9 + i * 9, rows.data() + i * kAtomVirW, 9 * sizeof(float));
 }
 
 }  // namespace b2m
@@ -1399,6 +1443,15 @@ int b2m_compute(b2m_handle h, int want_forces, int want_stress, double* energy, 
   API_END
 }
 
+int b2m_compute_peratom(b2m_handle h, int want_forces, double* energy, float* forces, float* stress9,
+                        double* atom_energy, float* atom_virial9) {
+  API_BEGIN
+  run_any(h, true, true);
+  fetch(h, energy, want_forces ? forces : nullptr, stress9);
+  fetch_peratom(h, atom_energy, atom_virial9);
+  API_END
+}
+
 int b2m_compute_resident(b2m_handle h, int want_forces, int want_stress, int reps, double* energy, float* ms) {
   API_BEGIN
   B2M_REQUIRE(reps >= 1, B2M_ERR_INVALID, "reps >= 1");
@@ -1539,8 +1592,10 @@ int b2m_release_workspace(b2m_handle h) {
     for (auto* b : {&e->be_e, &e->dbe_e, &e->Ha, &e->Hb, &e->Xc, &e->agg, &e->aggB, &e->y1p, &e->y1, &e->y2p, &e->y2,
                     &e->e_atom, &e->site, &e->gx, &e->gh, &e->gang, &e->gA, &e->gC, &e->gQ, &e->gHa, &e->gHb, &e->gXc,
                     &e->gagg, &e->gupd, &e->gaggB, &e->gd, &e->gdb, &e->gbvec, &e->gy1, &e->gy2, &e->forces,
-                    &e->sendbuf, &e->recvbuf, &e->site_full, &e->precv[0], &e->precv[1], &e->ftmp})
+                    &e->sendbuf, &e->recvbuf, &e->site_full, &e->precv[0], &e->precv[1], &e->ftmp, &e->atom_vir,
+                    &e->avtmp})
       drop(*b);
+    drop(e->atom_e), drop(e->aetmp);
     tn_release(e);
     e->g.~Graph();  // the resident graph goes too
     new (&e->g) Graph();

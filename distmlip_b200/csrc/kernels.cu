@@ -2,6 +2,7 @@
 // cp.async.bulk (TMA) row gathers into shared memory, segmented scatter-adds).
 // See kernels.cuh for the formulation; oracle/manual_ref.py is the CPU mirror of every stage.
 #include "kernels.cuh"
+#include "peratom.cuh"
 
 namespace b2m {
 
@@ -1272,6 +1273,23 @@ void launch_readout_seed(cudaStream_t st, int n, const float* pre, const float* 
   B2M_CK(cudaGetLastError());
   g_launch_count++;
 }
+__global__ void k_atom_energy(int n, const float* __restrict__ e_atom, const int* __restrict__ gid,
+                              const int* __restrict__ type, const double* __restrict__ elem_ref, float scale,
+                              double mean_per_atom, double* __restrict__ out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  // the same terms, in the same precision, as k_rowdot's / k_tn_readout_final's contribution to the energy
+  double v = (double)scale * (double)e_atom[i];
+  if (elem_ref) v += elem_ref[type[i]];
+  out[gid[i]] = v + mean_per_atom;
+}
+void launch_atom_energy(cudaStream_t st, int n_own, const float* e_atom, const int* gid, const int* type,
+                        const double* elem_ref, float scale, double mean_per_atom, double* out) {
+  if (n_own <= 0) return;
+  k_atom_energy<<<cdiv(n_own, 256), 256, 0, st>>>(n_own, e_atom, gid, type, elem_ref, scale, mean_per_atom, out);
+  B2M_CK(cudaGetLastError());
+  g_launch_count++;
+}
 
 // ============================================================================================
 // final geometry backward: forces and virial
@@ -1292,16 +1310,19 @@ __device__ __forceinline__ void virial_reduce(const float (&v)[9], double* __res
   }
 }
 
+// kPerAtom: also W_i (peratom.cuh) into atom_vir; the false instance is the plain kernel (atom_vir unused)
+template <bool kPerAtom>
 __global__ void __launch_bounds__(256) k_edge_final(int64_t E, const int* __restrict__ e_src,
                                                     const int* __restrict__ e_dst, const int* __restrict__ e_bond,
                                                     const float4* __restrict__ e_vec, const int* __restrict__ gid,
                                                     const float* __restrict__ gd, const float* __restrict__ gdb,
                                                     const float* __restrict__ gbvec, float* __restrict__ forces,
-                                                    double* __restrict__ virial) {
+                                                    double* __restrict__ virial, float* __restrict__ atom_vir) {
   const int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   float vir[9];
 #pragma unroll
   for (int k = 0; k < 9; k++) vir[k] = 0.f;
+  int pa_dst = -1, pa_src = 0;
   if (e < E) {
     const float4 v = e_vec[e];
     float g = gd[e];
@@ -1315,6 +1336,7 @@ __global__ void __launch_bounds__(256) k_edge_final(int64_t E, const int* __rest
     gx += s * v.x, gy += s * v.y, gz += s * v.z;
     // vec = x_dst + off.L - x_src :  dE/dx_dst += g, dE/dx_src -= g ; F = -dE/dx   (pes.py:122-124)
     const int gdst = gid[e_dst[e]], gsrc = gid[e_src[e]];
+    if constexpr (kPerAtom) pa_dst = gdst, pa_src = gsrc;
     atomicAdd(&forces[(size_t)gdst * 3], -gx);
     atomicAdd(&forces[(size_t)gdst * 3 + 1], -gy);
     atomicAdd(&forces[(size_t)gdst * 3 + 2], -gz);
@@ -1326,22 +1348,30 @@ __global__ void __launch_bounds__(256) k_edge_final(int64_t E, const int* __rest
     vir[3] = v.y * gx, vir[4] = v.y * gy, vir[5] = v.y * gz;
     vir[6] = v.z * gx, vir[7] = v.z * gy, vir[8] = v.z * gz;
   }
+  if constexpr (kPerAtom) atom_vir_edge(atom_vir, pa_dst, pa_src, vir);
   virial_reduce(vir, virial);
 }
 void launch_edge_final(cudaStream_t st, int64_t E, const int* e_src, const int* e_dst, const int* e_bond,
                        const float4* e_vec, const int* gid, const float* gd, const float* gdb, const float* gbvec,
-                       float* forces, double* virial) {
+                       float* forces, double* virial, float* atom_vir) {
   if (E <= 0) return;
-  k_edge_final<<<cdiv(E, 256), 256, 0, st>>>(E, e_src, e_dst, e_bond, e_vec, gid, gd, gdb, gbvec, forces, virial);
+  if (atom_vir)
+    k_edge_final<true><<<cdiv(E, 256), 256, 0, st>>>(E, e_src, e_dst, e_bond, e_vec, gid, gd, gdb, gbvec, forces,
+                                                     virial, atom_vir);
+  else
+    k_edge_final<false><<<cdiv(E, 256), 256, 0, st>>>(E, e_src, e_dst, e_bond, e_vec, gid, gd, gdb, gbvec, forces,
+                                                      virial, nullptr);
   B2M_CK(cudaGetLastError());
   g_launch_count++;
 }
 
+// kPerAtom: also W_i of both endpoints, per thread (halo bonds are few)
+template <bool kPerAtom>
 __global__ void __launch_bounds__(256) k_halo_bond_final(int b0, int b1, const int* __restrict__ b_src_gid,
                                                          const int* __restrict__ b_dst, const float4* __restrict__ b_vec,
                                                          const int* __restrict__ gid, const float* __restrict__ gdb,
                                                          const float* __restrict__ gbvec, float* __restrict__ forces,
-                                                         double* __restrict__ virial) {
+                                                         double* __restrict__ virial, float* __restrict__ atom_vir) {
   const int b = b0 + blockIdx.x * blockDim.x + threadIdx.x;
   float vir[9];
 #pragma unroll
@@ -1361,15 +1391,23 @@ __global__ void __launch_bounds__(256) k_halo_bond_final(int b0, int b1, const i
     vir[0] = v.x * gx, vir[1] = v.x * gy, vir[2] = v.x * gz;
     vir[3] = v.y * gx, vir[4] = v.y * gy, vir[5] = v.y * gz;
     vir[6] = v.z * gx, vir[7] = v.z * gy, vir[8] = v.z * gz;
+    if constexpr (kPerAtom) {
+      atom_vir_add(atom_vir, gdst, vir, 0.5f);
+      atom_vir_add(atom_vir, gsrc, vir, 0.5f);
+    }
   }
   virial_reduce(vir, virial);
 }
 void launch_halo_bond_final(cudaStream_t st, int b0, int b1, const int* b_src_gid, const int* b_dst,
                             const float4* b_vec, const int* gid, const float* gdb, const float* gbvec, float* forces,
-                            double* virial) {
+                            double* virial, float* atom_vir) {
   if (b1 <= b0) return;
-  k_halo_bond_final<<<cdiv(b1 - b0, 256), 256, 0, st>>>(b0, b1, b_src_gid, b_dst, b_vec, gid, gdb, gbvec, forces,
-                                                        virial);
+  if (atom_vir)
+    k_halo_bond_final<true><<<cdiv(b1 - b0, 256), 256, 0, st>>>(b0, b1, b_src_gid, b_dst, b_vec, gid, gdb, gbvec,
+                                                                forces, virial, atom_vir);
+  else
+    k_halo_bond_final<false><<<cdiv(b1 - b0, 256), 256, 0, st>>>(b0, b1, b_src_gid, b_dst, b_vec, gid, gdb, gbvec,
+                                                                 forces, virial, nullptr);
   B2M_CK(cudaGetLastError());
   g_launch_count++;
 }

@@ -132,14 +132,21 @@ void launch_rowdot(cudaStream_t st, int n, const float* X, const float* w, float
                    const int* type, const double* elem_ref, float scale);
 // g[r][c] = scale * w[c] * dsilu(pre[r][c])
 void launch_readout_seed(cudaStream_t st, int n, const float* pre, const float* w, float scale, float* g);
+// per-atom energy of the owned rows, in global order: out[gid[i]] = scale * e_atom[i] + elem_ref[type[i]] + mean_per_atom
+// (scale is the f32 data_std the energy sum uses, so that sum_i out[i] is the energy of the same evaluation)
+void launch_atom_energy(cudaStream_t st, int n_own, const float* e_atom, const int* gid, const int* type,
+                        const double* elem_ref, float scale, double mean_per_atom, double* out);
 
 // -------- final geometry backward --------
+// atom_vir: NULL (forces and total virial only), or [N][kAtomVirW] rows that also receive the per-atom virial
+// (peratom.cuh); the per-atom instances leave forces and the total virial exactly as the plain ones compute them
+constexpr int kAtomVirW = 12;
 void launch_edge_final(cudaStream_t st, int64_t E, const int* e_src, const int* e_dst, const int* e_bond,
                        const float4* e_vec, const int* gid, const float* gd, const float* gdb, const float* gbvec,
-                       float* forces /*[N,3]*/, double* virial /*[9]*/);
+                       float* forces /*[N,3]*/, double* virial /*[9]*/, float* atom_vir = nullptr);
 void launch_halo_bond_final(cudaStream_t st, int b0, int b1, const int* b_src_gid, const int* b_dst,
                             const float4* b_vec, const int* gid, const float* gdb, const float* gbvec, float* forces,
-                            double* virial);
+                            double* virial, float* atom_vir = nullptr);
 
 // -------- halo pack / unpack --------
 void launch_gather_rows(cudaStream_t st, int n, int width, const int* idx, const float* src, float* dst);
@@ -250,5 +257,5 @@ void launch_tn_readout_seed(cudaStream_t st, int n, int W, const float* lout, co
                             float* gG);
 void launch_tn_edge_final(cudaStream_t st, int64_t E, const int* e_src, const int* e_dst, const float4* e_vec,
                           const int* gid, const TnRadial& rp, const float* g_rbf, const float* gC, const float* gvh,
-                          float* gd, float* forces, double* virial);
+                          float* gd, float* forces, double* virial, float* atom_vir = nullptr);
 }  // namespace b2m

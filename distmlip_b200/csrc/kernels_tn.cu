@@ -17,6 +17,7 @@
 #include <math_constants.h>
 
 #include "kernels.cuh"
+#include "peratom.cuh"
 
 namespace b2m {
 
@@ -651,16 +652,20 @@ __device__ __forceinline__ void virial_reduce_tn(const float (&v)[9], double* __
     atomicAdd(&virial[threadIdx.x], s);
   }
 }
+// kPerAtom: also W_i (peratom.cuh) into atom_vir; the false instance is the plain kernel (atom_vir unused)
+template <bool kPerAtom>
 __global__ void __launch_bounds__(256) k_tn_edge_final(int64_t E, const int* __restrict__ e_src,
                                                        const int* __restrict__ e_dst, const float4* __restrict__ e_vec,
                                                        const int* __restrict__ gid, TnRadial rp,
                                                        const float* __restrict__ g_rbf, const float* __restrict__ gC,
                                                        const float* __restrict__ gvh, float* __restrict__ gd_out,
-                                                       float* __restrict__ forces, double* __restrict__ virial) {
+                                                       float* __restrict__ forces, double* __restrict__ virial,
+                                                       float* __restrict__ atom_vir) {
   const int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   float vir[9];
 #pragma unroll
   for (int k = 0; k < 9; k++) vir[k] = 0.f;
+  int pa_dst = -1, pa_src = 0;
   if (e < E) {
     const float4 v = e_vec[e];
     const float d = v.w, rd = 1.f / d;
@@ -677,6 +682,7 @@ __global__ void __launch_bounds__(256) k_tn_edge_final(int64_t E, const int* __r
     const float gx = gd * x + (hx - pr * x) * rd, gy = gd * y + (hy - pr * y) * rd, gz = gd * z + (hz - pr * z) * rd;
     // vec = x_dst + off.L - x_src :  dE/dx_dst += g, dE/dx_src -= g ; F = -dE/dx   (pes.py:122-124)
     const int gdst = gid[e_dst[e]], gsrc = gid[e_src[e]];
+    if constexpr (kPerAtom) pa_dst = gdst, pa_src = gsrc;
     atomicAdd(&forces[(size_t)gdst * 3], -gx);
     atomicAdd(&forces[(size_t)gdst * 3 + 1], -gy);
     atomicAdd(&forces[(size_t)gdst * 3 + 2], -gz);
@@ -687,6 +693,7 @@ __global__ void __launch_bounds__(256) k_tn_edge_final(int64_t E, const int* __r
     vir[3] = v.y * gx, vir[4] = v.y * gy, vir[5] = v.y * gz;
     vir[6] = v.z * gx, vir[7] = v.z * gy, vir[8] = v.z * gz;
   }
+  if constexpr (kPerAtom) atom_vir_edge(atom_vir, pa_dst, pa_src, vir);
   virial_reduce_tn(vir, virial);
 }
 
@@ -782,8 +789,11 @@ void launch_tn_readout_seed(cudaStream_t st, int n, int W, const float* lout, co
 }
 void launch_tn_edge_final(cudaStream_t st, int64_t E, const int* e_src, const int* e_dst, const float4* e_vec,
                           const int* gid, const TnRadial& rp, const float* g_rbf, const float* gC, const float* gvh,
-                          float* gd, float* forces, double* virial) {
-  TN_LAUNCH(k_tn_edge_final, E, st, E, e_src, e_dst, e_vec, gid, rp, g_rbf, gC, gvh, gd, forces, virial);
+                          float* gd, float* forces, double* virial, float* atom_vir) {
+  if (atom_vir)
+    TN_LAUNCH(k_tn_edge_final<true>, E, st, E, e_src, e_dst, e_vec, gid, rp, g_rbf, gC, gvh, gd, forces, virial, atom_vir);
+  else
+    TN_LAUNCH(k_tn_edge_final<false>, E, st, E, e_src, e_dst, e_vec, gid, rp, g_rbf, gC, gvh, gd, forces, virial, nullptr);
 }
 
 }  // namespace b2m

@@ -29,6 +29,8 @@ class Distributed:
         self.total_num_edges = None  # global count needs a reduction over ranks; see num_atom_edges
         self.forces = None
         self.stress = None
+        self.energies = None  # per-atom energies [N] (eV) and stresses [N,3,3] (GPa) of a calc_per_atom evaluation
+        self.stresses = None
 
     @staticmethod
     def cartesian_to_wrapped_fractional(positions_cartesian, lattice, pbc):

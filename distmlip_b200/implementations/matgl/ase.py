@@ -29,9 +29,10 @@ except Exception:  # noqa: BLE001
 
 
 def _voigt6(s):
+    """[..., 3, 3] -> [..., 6] (xx, yy, zz, yz, xz, xy)"""
     s = np.asarray(s)
-    return np.array([s[0, 0], s[1, 1], s[2, 2], (s[1, 2] + s[2, 1]) / 2, (s[0, 2] + s[2, 0]) / 2,
-                     (s[0, 1] + s[1, 0]) / 2])
+    return np.stack([s[..., 0, 0], s[..., 1, 1], s[..., 2, 2], (s[..., 1, 2] + s[..., 2, 1]) / 2,
+                     (s[..., 0, 2] + s[..., 2, 0]) / 2, (s[..., 0, 1] + s[..., 1, 0]) / 2], axis=-1)
 
 
 class PESCalculator_Dist(_Calculator):
@@ -47,6 +48,9 @@ class PESCalculator_Dist(_Calculator):
         self.compute_stress = potential.calc_stresses
         self.compute_hessian = potential.calc_hessian
         self.compute_magmom = potential.calc_site_wise
+        self.compute_per_atom = getattr(potential, "calc_per_atom", False)
+        if self.compute_per_atom:  # ASE's per-atom properties, offered when the potential computes them
+            self.implemented_properties = type(self).implemented_properties + ("energies", "stresses")
         if stress_unit == "eV/A3":
             conversion_factor = 0.006241509125883258  # GPa -> eV/A^3 (ase.units)
         elif stress_unit == "GPa":
@@ -74,6 +78,11 @@ class PESCalculator_Dist(_Calculator):
             self.results.update(stress=(_voigt6(st) if self.use_voigt else st) * self.stress_weight)
         if self.compute_magmom:
             self.results.update(magmoms=calc_result[4].detach().cpu().numpy())
+        if self.compute_per_atom:  # ASE's per-atom properties: they sum to `energy` and `stress`
+            info = self.potential.last_dist_info
+            sts = np.asarray(info.stresses)
+            self.results.update(energies=np.asarray(info.energies),
+                                stresses=(_voigt6(sts) if self.use_voigt else sts) * self.stress_weight)
 
 
 class TrajectoryObserver:

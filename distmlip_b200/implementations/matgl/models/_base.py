@@ -123,11 +123,18 @@ class EngineBackedModel:
     def potential_forward_dist(self, dist_info, atoms, lattice_matrix, calc_stresses, calc_forces, calc_hessian,
                                state_attr=None):
         """Seam of chgnet.py:21-30,199-206 / tensornet.py:10-19.  Returns (node_types, positions, strain, (E, site_wise));
-        forces / stress of the same evaluation are left on `dist_info` (no autograd graph exists)."""
+        forces / stress of the same evaluation are left on `dist_info` (no autograd graph exists), and so are the
+        per-atom energies [N] (eV) and stresses [N,3,3] (GPa, W_i * 160.21766208 / V) when the Potential asks for them."""
         if calc_hessian:
             raise NotImplementedError("Calculating hessians is not implemented for distributed inference.")
         eng = self._engine
-        e, f, s = eng.compute(forces=calc_forces, stress=calc_stresses)
+        if self.__dict__.get("_want_peratom", False):
+            e, f, s, atom_e, atom_w = eng.compute_peratom(forces=calc_forces)
+            s = s if calc_stresses else None
+            dist_info.energies = atom_e
+            dist_info.stresses = atom_w * (160.21766208 / abs(np.linalg.det(np.asarray(lattice_matrix, dtype=float))))
+        else:
+            e, f, s = eng.compute(forces=calc_forces, stress=calc_stresses)
         dist_info.forces, dist_info.stress = f, s
         node_types = torch.as_tensor(dist_info.species, dtype=distmlip_b200.int_th)
         positions = torch.from_numpy(dist_info.cart)  # zero-copy view (f64); no autograd graph hangs off it here

@@ -5,6 +5,10 @@ Same constructor kwargs and call convention: `potential(atoms, state_attr=None, 
 deliberate: one partition is allowed (the reference asserts > 1 GPU, pes.py:40-42); energy, forces and
 stress come out of one b2m_compute call (hand-written backward) instead of torch.autograd.backward
 (pes.py:122-124); results are CPU tensors (the ASE calculator immediately calls .cpu().numpy()).
+
+`calc_per_atom=True` (not in the reference) also computes per-atom energies and stresses in the same evaluation and leaves
+them on `last_dist_info` as `energies` [N] (eV) and `stresses` [N,3,3] (GPa); they sum to the energy and the stress.
+The return tuple does not change.
 """
 from __future__ import annotations
 
@@ -23,7 +27,7 @@ class Potential_Dist:
 
     def __init__(self, model=None, num_threads=None, data_mean=0.0, data_std=1.0, element_refs=None,
                  calc_forces=True, calc_stresses=True, calc_hessian=False, calc_site_wise=False, debug_mode=False,
-                 calc_repuls=False, zbl_trainable=False, **kwargs):
+                 calc_repuls=False, zbl_trainable=False, calc_per_atom=False, **kwargs):
         if model is None:
             raise ValueError("model is required")
         self.model = model
@@ -35,6 +39,7 @@ class Potential_Dist:
         self.calc_stresses = calc_stresses
         self.calc_hessian = calc_hessian
         self.calc_site_wise = calc_site_wise
+        self.calc_per_atom = calc_per_atom
         self.debug_mode = debug_mode
         self.data_mean = float(torch.as_tensor(data_mean).item()) if data_mean is not None else 0.0
         self.data_std = float(torch.as_tensor(data_std).item()) if data_std is not None else 1.0
@@ -62,6 +67,7 @@ class Potential_Dist:
         model = self.model
         species = model._species_of(atoms)
         model._want_site = bool(self.calc_site_wise)
+        model._want_peratom = bool(self.calc_per_atom)
         model._finalize(self.data_mean, self.data_std, self.element_refs)
         dist_info = Distributed.create_distributed(
             cart_coords=cart_coords, frac_coords=None, lattice_matrix=lattice_matrix,

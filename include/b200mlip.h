@@ -122,6 +122,17 @@ int b2m_set_structure(b2m_handle h, int64_t natoms, const double* cart, const do
 /* Energy (+forces [natoms,3] eV/A, +stress [9] GPa).  forces/stress9 may be NULL.
  * With world > 1 every rank receives the full (all-reduced) result. */
 int b2m_compute(b2m_handle h, int want_forces, int want_stress, double* energy, float* forces, float* stress9);
+/* b2m_compute (energy, forces if want_forces, stress) plus per-atom output of the same evaluation.  CHGNet and
+ * TensorNet handles, every process model; atom_energy / atom_virial9 may be NULL.  For N atoms and cell volume V:
+ *   atom_energy [natoms] f64, eV:   e_i = data_std * e^_i + element_ref[type_i] + data_mean / N
+ *        (e^_i: the model's raw per-atom output); sum_i e_i = energy of the same call.
+ *   atom_virial9 [natoms,9] f32, eV, row-major 3x3, not symmetrised:
+ *        W_i[a][b] = 1/2 sum_{e : src(e)=i or dst(e)=i} vec_e[a] g_e[b],
+ *        vec_e = x_dst + off.L - x_src, g_e = dE/dvec_e (each edge's term split evenly between its two atoms);
+ *        sum_i W_i = dE/dstrain, so sum_i W_i * 160.21766208 / V = stress9 (GPa) of the same call.
+ * The per-atom buffers (56 B per atom and partition) are allocated by the first such call. */
+int b2m_compute_peratom(b2m_handle h, int want_forces, double* energy, float* forces, float* stress9,
+                        double* atom_energy /* [natoms] or NULL */, float* atom_virial9 /* [natoms,9] eV or NULL */);
 /* Same arithmetic, graph already resident; runs `reps` passes and returns device time (ms) of
  * the last one measured with CUDA events on the compute stream. Used by bench.py `value`. */
 int b2m_compute_resident(b2m_handle h, int want_forces, int want_stress, int reps, double* energy, float* ms);
